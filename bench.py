@@ -25,6 +25,7 @@ if ROOT not in sys.path:
 
 BASELINE_PUBLISHED = None   # the reference publishes no throughput number (BASELINE.md §1)
 BERT_MODELS = ("bert", "bert_large", "bert_base")
+DUMP_STATE_SAMPLE = 1 << 22      # --dump-outputs: 16 MB of float32; >= 1 % of BERT-large's 336 M elements
 
 
 def parse_args(argv=None):
@@ -62,7 +63,14 @@ def parse_args(argv=None):
                     help="end-to-end run: spin this long on the copy stream before each prefetch upload so the PCIe DMA does "
                          "not start at the step boundary, where the rotated step runs the update + all-gather kernels "
                          "(utils/data.py). Default: 2000 with --overlap-update 1, else 0")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed (rank 0) as float32 .npy files: "
+                         "loss.npy, and model_state.npy, the floating-point entries of the model's state_dict with that "
+                         "step's update applied, flattened in state_dict order (a fixed sample of %d elements when larger)"
+                         % DUMP_STATE_SAMPLE)
     args = ap.parse_args(argv)
+    if args.dump_outputs and (args.impl != "dear" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl dear and --steps >= 1")
     is_bert = args.model in BERT_MODELS
     if args.batch_size is None:
         args.batch_size = 32 if is_bert else 64
@@ -244,12 +252,19 @@ def run_dear(args):
         dear.barrier()
         return ms, n_launches() - l0
 
+    last_loss = [None]
+
+    def resident():
+        last_loss[0] = step(*dev_batch)
+
     sampler = ClockSampler(device.index if cuda else 0).start() if (cuda and rank == 0) else None
     wall0 = time.time()
-    ms, launches = timed(lambda: step(*dev_batch), args.steps)
+    ms, launches = timed(resident, args.steps)
     wall1 = time.time()
     if args.graph and cuda:
         launches = int(round(per_step_launches * args.steps))
+    if args.dump_outputs:
+        _dump_outputs(args.dump_outputs, last_loss[0], opt, model, rank)
 
     # ---- end to end: pinned host batches -> H2D every step, loss -> host every step ----------
     e2e = None
@@ -314,6 +329,25 @@ def run_dear(args):
         traceback.print_exc()
     dear.shutdown()
     return 0
+
+
+def _dump_outputs(path, loss, opt, model, rank):
+    """--dump-outputs: the loss of the last timed step and the model state after its update."""
+    import numpy as np
+    import torch
+    loss = loss.detach().float().cpu().reshape(1)   # before synchronize(): a replayed graph reuses this buffer
+    opt.synchronize()                               # rotated step: applies the update of the last call, on every rank
+    if rank != 0:
+        return
+    state = torch.cat([t.detach().reshape(-1).float() for t in model.state_dict().values() if t.is_floating_point()])
+    if state.numel() > DUMP_STATE_SAMPLE:             # one seeded random element from each of DUMP_STATE_SAMPLE equal slices
+        edges = torch.arange(DUMP_STATE_SAMPLE + 1, dtype=torch.int64) * state.numel() // DUMP_STATE_SAMPLE
+        u = torch.rand(DUMP_STATE_SAMPLE, generator=torch.Generator().manual_seed(0), dtype=torch.float64)
+        idx = edges[:-1] + (u * (edges[1:] - edges[:-1])).long()
+        state = state[idx.to(state.device)]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "loss.npy"), loss.numpy())
+    np.save(os.path.join(path, "model_state.npy"), state.cpu().numpy())
 
 
 def _max_over_ranks(v, world):

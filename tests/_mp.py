@@ -39,12 +39,18 @@ def _worker(rank, world, port, backend, fn, args, ret, extra_env):
 def run_ranks(fn, world=2, backend="gloo", args=(), timeout=240, extra_env=None, start_method=None):
     """Run ``fn(rank, world, *args)`` on ``world`` processes; returns the list of results.
 
-    CPU backends fork (the children inherit the already-imported torch: ~10x faster than spawn);
-    anything touching CUDA must spawn.
+    CPU backends start their ranks from a fork server that has imported torch but never run autograd (~10x faster
+    than spawn).  Forking the test process itself is not safe: once it has run a backward pass on a machine with a
+    GPU, autograd's per-device worker threads exist and a forked child's backward raises.  Anything touching CUDA
+    must spawn.  Either way ``fn`` and ``args`` are pickled, so ``fn`` must be a module-level function.
     """
     if start_method is None:
-        start_method = "fork" if backend in ("gloo", "emu") and not torch.cuda.is_initialized() else "spawn"
+        start_method = "forkserver" if backend in ("gloo", "emu") else "spawn"
     ctx = mp.get_context(start_method)
+    if start_method == "forkserver":
+        # takes effect when the (per test session) server starts; the first torch.optim optimizer of a process imports
+        # torch._dynamo, which costs seconds per rank unless the server did it once
+        ctx.set_forkserver_preload(["torch", "torch._dynamo"])
     mgr = ctx.Manager()
     ret = mgr.dict()
     port = free_port()

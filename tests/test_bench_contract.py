@@ -37,6 +37,25 @@ def test_bench_two_ranks_native_emulation():
     assert d["gpu_launches"] == 2 * 2 * d["config"]["buckets"]      # one RS + one AG per bucket per step
 
 
+def test_dump_outputs_are_float32_bounded_and_reproducible(tmp_path):
+    import numpy as np
+    args = ["--backend", "gloo", "--model", "resnet18", "--batch-size", "2", "--warmup", "1", "--no-e2e"]
+    dumps = []
+    for name, steps in (("a", 2), ("b", 2), ("c", 3)):
+        # on the CPU even where a GPU is present: cuDNN's autotuner may pick other algorithms from run to run
+        run(args + ["--steps", str(steps), "--dump-outputs", str(tmp_path / name)], env={"CUDA_VISIBLE_DEVICES": ""})
+        files = sorted(os.listdir(tmp_path / name))
+        assert files == ["loss.npy", "model_state.npy"]
+        arrays = {f: np.load(tmp_path / name / f) for f in files}
+        assert all(a.dtype == np.float32 for a in arrays.values())
+        assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+        assert arrays["loss.npy"].shape == (1,) and np.isfinite(arrays["loss.npy"]).all()
+        dumps.append(arrays)
+    for f in dumps[0]:
+        np.testing.assert_array_equal(dumps[0][f], dumps[1][f])       # same arguments: same inputs, same outputs
+        assert not np.array_equal(dumps[0][f], dumps[2][f])           # one more timed step: another loss and state
+
+
 def test_reference_arm_reports_unavailable_without_gpu():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference"], cwd=ROOT,
                          capture_output=True, text=True, timeout=300)

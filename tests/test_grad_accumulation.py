@@ -121,19 +121,21 @@ def test_parameter_used_in_only_some_passes(backend):
             torch.testing.assert_close(a, b.detach(), rtol=5e-5, atol=5e-6)
 
 
-def test_second_backward_without_accumulation_is_an_error():
-    def w(rank, world):
-        import dear_pytorch_b200 as dear
-        model = make_model(); model.eval()
-        opt = dear.DistributedOptimizer(torch.optim.SGD(model.parameters(), lr=0.1), model, threshold=0.001, verbose=False)
-        x, y = data(0, 4)
+def _second_backward_worker(rank, world):
+    import dear_pytorch_b200 as dear
+    model = make_model(); model.eval()
+    opt = dear.DistributedOptimizer(torch.optim.SGD(model.parameters(), lr=0.1), model, threshold=0.001, verbose=False)
+    x, y = data(0, 4)
+    nn.functional.cross_entropy(model(x), y).backward()
+    try:
         nn.functional.cross_entropy(model(x), y).backward()
-        try:
-            nn.functional.cross_entropy(model(x), y).backward()
-        except RuntimeError as e:
-            return "backward_passes_per_step" in str(e)
-        return False
-    assert all(run_ranks(w, world=1, backend="gloo"))
+    except RuntimeError as e:
+        return "backward_passes_per_step" in str(e)
+    return False
+
+
+def test_second_backward_without_accumulation_is_an_error():
+    assert all(run_ranks(_second_backward_worker, world=1, backend="gloo"))
 
 
 def _intermittent_worker(rank, world, steps, k, per):

@@ -58,12 +58,14 @@ def test_norm_clip_matches_clip_grad_norm(backend, world, kind, clip):
             torch.testing.assert_close(a, b, rtol=2e-5, atol=2e-6)
 
 
+def _zero_clip_worker(rank, world):
+    import dear_pytorch_b200 as dear
+    m = nn.Linear(2, 2)
+    try:
+        dear.DistributedOptimizer(torch.optim.SGD(m.parameters(), lr=0.1), m, norm_clip=0.0, verbose=False)
+    except ValueError as e:
+        return str(e)
+
+
 def test_norm_clip_rejects_nonsense():
-    def w(rank, world):
-        import dear_pytorch_b200 as dear
-        m = nn.Linear(2, 2)
-        try:
-            dear.DistributedOptimizer(torch.optim.SGD(m.parameters(), lr=0.1), m, norm_clip=0.0, verbose=False)
-        except ValueError as e:
-            return str(e)
-    assert all("positive" in (o or "") for o in run_ranks(w, world=2, backend="emu"))
+    assert all("positive" in (o or "") for o in run_ranks(_zero_clip_worker, world=2, backend="emu"))

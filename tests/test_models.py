@@ -125,30 +125,41 @@ def test_cnn_matches_torchvision(name):
             torch.testing.assert_close(va, vb, rtol=1e-5, atol=1e-6)      # the training forward updated the same statistics
 
 
+def seeded_state_dict(sd):
+    """Deterministic values for a state dict, drawn in its order from its shapes and attribute names only, so two modules
+    whose tensors line up one to one receive the same values: He-scaled convolution / linear weights, non-trivial
+    BatchNorm statistics and affine parameters."""
+    g = torch.Generator().manual_seed(0)
+    out = {}
+    for k, v in sd.items():
+        if not v.is_floating_point():
+            out[k] = v.clone()
+        elif v.dim() > 1:
+            out[k] = torch.randn(v.shape, generator=g) * (2.0 / v[0].numel()) ** 0.5
+        elif k.endswith(("running_var", "weight")):
+            out[k] = torch.rand(v.shape, generator=g) + 0.5
+        else:
+            out[k] = torch.randn(v.shape, generator=g) * 0.1
+    return out
+
+
+def inceptionv4_input():
+    return torch.randn(2, 3, 299, 299, generator=torch.Generator().manual_seed(1))
+
+
 def test_inceptionv4_matches_the_reference_file():
-    """The reference ships its own Inception-v4 (dear/inceptionv4.py, the Cadene implementation).  When the reference arm
-    is installed (baseline/_ref, used by `bench.py --impl reference`), load its class next to ours: the tensors line up one
-    to one (896, same order and shapes) and the function is the same."""
-    import glob
-    import importlib.util
+    """The reference ships its own Inception-v4 (dear/inceptionv4.py, the Cadene implementation).  Its tensors line up
+    with ours one to one (896, same order and shapes), and with the same values both compute the same function.  The
+    reference's shapes and its logits for seeded weights and inputs are stored in tests/golden/ (written by
+    tests/golden/make_inceptionv4_reference.py)."""
+    import json
     import os
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    found = glob.glob(os.path.join(root, "baseline", "_ref", "dear", "inceptionv4.py"))
-    if not found:
-        pytest.skip("reference arm not installed (baseline/_ref)")
-    spec = importlib.util.spec_from_file_location("_ref_inceptionv4", found[0])
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    torch.manual_seed(0)
-    ref = mod.InceptionV4(num_classes=1000).eval()
-    with torch.no_grad():
-        for m in ref.modules():
-            if isinstance(m, torch.nn.BatchNorm2d):
-                m.running_mean.normal_(0, 0.1); m.running_var.uniform_(0.5, 1.5); m.weight.uniform_(0.5, 1.5); m.bias.normal_(0, 0.1)
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "inceptionv4_reference.json")) as f:
+        golden = json.load(f)
     ours = create("inceptionv4").eval()
-    mine, src = ours.state_dict(), ref.state_dict()
-    assert [tuple(v.shape) for v in mine.values()] == [tuple(v.shape) for v in src.values()]
-    ours.load_state_dict(dict(zip(mine.keys(), src.values())))
-    x = torch.randn(1, 3, 299, 299)
+    mine = ours.state_dict()
+    assert len(mine) == 896
+    assert [list(v.shape) for v in mine.values()] == golden["state_dict_shapes"]
+    ours.load_state_dict(seeded_state_dict(mine))
     with torch.no_grad():
-        torch.testing.assert_close(ours(x), ref(x), rtol=1e-3, atol=1e-3)
+        torch.testing.assert_close(ours(inceptionv4_input()), torch.tensor(golden["logits"]), rtol=1e-3, atol=1e-3)

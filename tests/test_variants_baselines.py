@@ -82,21 +82,23 @@ def test_variant_matches_sgd(kind):
             assert max(n for _, _, n in log) <= partition and any(i > 0 for _, i, _ in log)   # tensors were partitioned
 
 
+def _wfbp_timers_worker(rank, world):
+    import dear_pytorch_b200 as dear
+    from dear_pytorch_b200.parallel.baselines import WFBPDistributedOptimizer
+    model = make_model()
+    opt = WFBPDistributedOptimizer(torch.optim.SGD(model.parameters(), lr=0.05), model=model, compression="topk",
+                                   is_sparse=True, density=0.25, threshold=600, profiling=True, verbose=False)
+    dear.broadcast_parameters(model.state_dict(), 0)
+    for t in range(2):
+        x, y = data(t, 8)
+        opt.zero_grad()
+        nn.functional.cross_entropy(model(x[rank * 4:(rank + 1) * 4]), y[rank * 4:(rank + 1) * 4]).backward()
+        opt.step()
+    return opt.profiling_summary()
+
+
 def test_wfbp_in_optimizer_timers():
-    def w(rank, world):
-        import dear_pytorch_b200 as dear
-        from dear_pytorch_b200.parallel.baselines import WFBPDistributedOptimizer
-        model = make_model()
-        opt = WFBPDistributedOptimizer(torch.optim.SGD(model.parameters(), lr=0.05), model=model, compression="topk",
-                                       is_sparse=True, density=0.25, threshold=600, profiling=True, verbose=False)
-        dear.broadcast_parameters(model.state_dict(), 0)
-        for t in range(2):
-            x, y = data(t, 8)
-            opt.zero_grad()
-            nn.functional.cross_entropy(model(x[rank * 4:(rank + 1) * 4]), y[rank * 4:(rank + 1) * 4]).backward()
-            opt.step()
-        return opt.profiling_summary()
-    out = run_ranks(w, world=2, backend="gloo")[0]
+    out = run_ranks(_wfbp_timers_worker, world=2, backend="gloo")[0]
     assert out["compression"] and set(out["compression"]) == set(out["allreduce"]) == set(out["update"])
     assert all(v > 0 for v in out["allreduce"].values())
 
@@ -125,49 +127,53 @@ def test_bytescheduler_priority_and_credit():
     assert order == [(0, 0), (0, 1), (2, 0), (2, 1), (5, 0), (5, 1), (5, 2), (7, 0)]
 
 
+def _sparse_consistency_worker(rank, world, compressor, mc):
+    import dear_pytorch_b200 as dear
+    from dear_pytorch_b200.parallel.baselines import WFBPDistributedOptimizer
+    model = make_model()
+    opt = torch.optim.SGD(model.parameters(), lr=0.05, momentum=0.9 if mc else 0.0)
+    opt = WFBPDistributedOptimizer(opt, model=model, compression=compressor, is_sparse=True, density=0.25,
+                                   threshold=10 ** 9, momentum_correction=mc, verbose=False)
+    dear.broadcast_parameters(model.state_dict(), 0)
+    losses = []
+    for t in range(8):
+        x, y = data(0, 8)
+        opt.zero_grad()
+        loss = nn.functional.cross_entropy(model(x[rank * 4:(rank + 1) * 4]), y[rank * 4:(rank + 1) * 4])
+        loss.backward()
+        opt.step()
+        losses.append(float(loss))
+    return losses, [p.detach().clone() for p in model.parameters()]
+
+
 @pytest.mark.parametrize("compressor,mc", [("gtopk", False), ("gtopkef", False), ("topk", True), ("gaussian", False)])
 def test_sparse_paths_stay_rank_consistent(compressor, mc):
-    def sparse_worker(rank, world, compressor, mc):
-        import dear_pytorch_b200 as dear
-        from dear_pytorch_b200.parallel.baselines import WFBPDistributedOptimizer
-        model = make_model()
-        opt = torch.optim.SGD(model.parameters(), lr=0.05, momentum=0.9 if mc else 0.0)
-        opt = WFBPDistributedOptimizer(opt, model=model, compression=compressor, is_sparse=True, density=0.25,
-                                       threshold=10 ** 9, momentum_correction=mc, verbose=False)
-        dear.broadcast_parameters(model.state_dict(), 0)
-        losses = []
-        for t in range(8):
-            x, y = data(0, 8)
-            opt.zero_grad()
-            loss = nn.functional.cross_entropy(model(x[rank * 4:(rank + 1) * 4]), y[rank * 4:(rank + 1) * 4])
-            loss.backward()
-            opt.step()
-            losses.append(float(loss))
-        return losses, [p.detach().clone() for p in model.parameters()]
-    outs = run_ranks(sparse_worker, world=2, backend="gloo", args=(compressor, mc))
+    outs = run_ranks(_sparse_consistency_worker, world=2, backend="gloo", args=(compressor, mc))
     assert all(torch.equal(a, b) for a, b in zip(outs[0][1], outs[1][1]))
     assert outs[0][0][-1] < outs[0][0][0]            # the sparsified run still trains
 
 
+def _sparse_topk_allgather_worker(rank, world):
+    import dear_pytorch_b200 as dear
+    from dear_pytorch_b200.parallel.baselines import WFBPDistributedOptimizer
+    model = make_model()
+    opt = torch.optim.SGD(model.parameters(), lr=0.05)
+    opt = WFBPDistributedOptimizer(opt, model=model, compression="topk", is_sparse=True, density=0.25, threshold=0,
+                                   verbose=False)
+    dear.broadcast_parameters(model.state_dict(), 0)
+    losses = []
+    for t in range(6):
+        x, y = data(0, 8)
+        opt.zero_grad()
+        loss = nn.functional.cross_entropy(model(x[rank * 4:(rank + 1) * 4]), y[rank * 4:(rank + 1) * 4])
+        loss.backward()
+        opt.step()
+        losses.append(float(loss))
+    return losses, [p.detach().clone() for p in model.parameters()]
+
+
 def test_sparse_topk_allgather_path_runs():
-    def sparse_worker(rank, world):
-        import dear_pytorch_b200 as dear
-        from dear_pytorch_b200.parallel.baselines import WFBPDistributedOptimizer
-        model = make_model()
-        opt = torch.optim.SGD(model.parameters(), lr=0.05)
-        opt = WFBPDistributedOptimizer(opt, model=model, compression="topk", is_sparse=True, density=0.25, threshold=0,
-                                       verbose=False)
-        dear.broadcast_parameters(model.state_dict(), 0)
-        losses = []
-        for t in range(6):
-            x, y = data(0, 8)
-            opt.zero_grad()
-            loss = nn.functional.cross_entropy(model(x[rank * 4:(rank + 1) * 4]), y[rank * 4:(rank + 1) * 4])
-            loss.backward()
-            opt.step()
-            losses.append(float(loss))
-        return losses, [p.detach().clone() for p in model.parameters()]
-    outs = run_ranks(sparse_worker, world=2, backend="gloo")
+    outs = run_ranks(_sparse_topk_allgather_worker, world=2, backend="gloo")
     assert all(torch.equal(a, b) for a, b in zip(outs[0][1], outs[1][1]))
     assert outs[0][0][-1] < outs[0][0][0] + 0.5
 
@@ -204,16 +210,18 @@ def test_horovod_adasum_adds_orthogonal_and_averages_parallel_gradients(world):
         assert all(torch.equal(a, b) for a, b in zip(outs[0], outs[-1]))       # bit-identical on every rank
 
 
+def _adasum_three_ranks_worker(rank, world):
+    from dear_pytorch_b200.parallel.baselines import HorovodOptimizer
+    m = nn.Linear(2, 2)
+    try:
+        HorovodOptimizer(torch.optim.SGD(m.parameters(), lr=1.0), m, op="adasum", verbose=False)
+    except ValueError as e:
+        return str(e)
+    return None
+
+
 def test_adasum_needs_a_power_of_two():
-    def w(rank, world):
-        from dear_pytorch_b200.parallel.baselines import HorovodOptimizer
-        m = nn.Linear(2, 2)
-        try:
-            HorovodOptimizer(torch.optim.SGD(m.parameters(), lr=1.0), m, op="adasum", verbose=False)
-        except ValueError as e:
-            return str(e)
-        return None
-    assert all("power-of-two" in (o or "") for o in run_ranks(w, world=3, backend="gloo"))
+    assert all("power-of-two" in (o or "") for o in run_ranks(_adasum_three_ranks_worker, world=3, backend="gloo"))
 
 
 def _fp16_worker(rank, world):

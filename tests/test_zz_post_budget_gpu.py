@@ -147,15 +147,15 @@ def test_baseline_methods_of_the_driver_over_nccl(method, extra):
 
 
 # ---- a slice of the randomised equivalence fuzzer on the fused kernels -----------------------------------------------------------
-def test_fuzz_slice_on_the_fused_kernels():
+def test_fuzz_slice_on_the_fused_kernels(monkeypatch):
     """tools/fuzz_equivalence.py with ``--backends b200``: random models / optimizers / bucketing / accumulation / re-bucketing /
     state-dict round trips / TrainStep bodies on the GPU data path against single-process torch.optim on the CPU."""
-    import importlib.util
+    import importlib
     import os
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    spec = importlib.util.spec_from_file_location("fuzz_equivalence_gpu", os.path.join(root, "tools", "fuzz_equivalence.py"))
-    fuzz = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(fuzz)
+    # CUDA ranks are spawned, not forked: they unpickle the fuzzer's worker by module name, so the module must be
+    # importable under its own name from a path the children inherit
+    monkeypatch.syspath_prepend(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
+    fuzz = importlib.import_module("fuzz_equivalence")
     failures = fuzz.main(["--seed", "5", "--trials", "6", "--backends", "b200", "--max-world", "2", "--quiet",
                           "--variants", "dear,dear,dear,bo,naive,wt,rb"])
     assert not failures, failures[0]
