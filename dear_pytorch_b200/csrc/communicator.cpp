@@ -736,8 +736,11 @@ void BucketSet::reduce_scatter(int g, bool pack) {
     p.segs = cuda ? table_dev : b.pack_host.data();
     p.nseg = static_cast<uint32_t>(b.pack_host.size());
     p.ntiles = b.ntiles;
-    // one GPU: the pack writes the fp32 shard directly (fp32: copy; bf16 / fp16: widening, CUDA kernel only)
-    p.direct_out = (comm_->size() == 1 && (dtype_ == DT_F32 || cuda) && !b.pack_inplace) ? 1u : 0u;
+    // one GPU: the pack writes the fp32 shard directly (fp32: copy; bf16 / fp16: widening, CUDA kernel only).  The
+    // fp32 copy cannot apply a gradient scale (1/loss_scale), so a scaled fp32 bucket packs into the gradient bucket
+    // and the reduce pass applies the scale.
+    const bool direct_ok = dtype_ == DT_F32 ? grad_scale_ == 1.f : cuda;
+    p.direct_out = (comm_->size() == 1 && direct_ok && !b.pack_inplace) ? 1u : 0u;
   }
   p.sig = arena_->sig_table();
   p.ctrl = arena_->ctrl();
